@@ -2,6 +2,7 @@
 """Benchmark of the PixelSSL sseg SSL-training hot path on B200.
 
     python bench.py --gpus N --steps K --warmup W [--config mt|cutmix|gct|cct] [--precision f16x3|f16|tf32x3|tf32|fp32]
+                    [--dump-outputs DIR]
     python bench.py --impl reference --gpus N --steps K --warmup W          (torchrun for N > 1)
 
 Default workload (BASELINE.json configs[1]): Mean-Teacher, DeepLab-v2-ResNet101 OS16, per-GPU batch 16
@@ -150,6 +151,31 @@ def synthetic_host_batches(count, rank, pin, lbs=None, ubs=None, size=None):
             img, lab = img.pin_memory(), lab.pin_memory()
         out.append((img, lab))
     return out
+
+
+DUMP_PARAM_BYTES = 60 * 2 ** 20          # model-state share of the 64 MB --dump-outputs budget
+
+
+def dump_outputs(alg, out_dir):
+    """What the last step of ``algorithm._train`` leaves its caller, as ``out_dir/<name>.npy``: every meter of the
+    step except the wall-clock ``batch_time`` (float64 scalar, e.g. ``s_task_loss.npy``) and, per model of
+    ``algorithm.models``, its floating-point state_dict entries in key order flattened to one float32 vector
+    (``s_model.npy``; parameters and BN running statistics).  Where the models together exceed DUMP_PARAM_BYTES, each
+    vector is a fixed sample of it: the same seeded, sorted indices in every run, so two builds compare element for
+    element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for key in sorted(alg.meters.keys()):
+        if key != 'batch_time':
+            np.save(os.path.join(out_dir, key + '.npy'), np.array(float(alg.meters[key].val), dtype=np.float64))
+    per_model = DUMP_PARAM_BYTES // 4 // len(alg.models)
+    for name, model in sorted(alg.models.items()):
+        flat = torch.cat([t.detach().reshape(-1).float() for t in model.state_dict().values() if t.is_floating_point()])
+        if flat.numel() > per_model:
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), per_model, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), flat.cpu().numpy())
 
 
 def _roofline_from(records, peak, src, kernel, bound='tensor', traffic=None):
@@ -330,6 +356,8 @@ def run_engine(args):
             clock_rec.append(sampler.stop())
         ms = e0.elapsed_time(e1)
         ktimes = ops.kernel_timer_stop('pxl_mse_consistency')
+        if tag == 'value' and args.dump_outputs and rank == 0:
+            dump_outputs(st['alg'], args.dump_outputs)
         if tag:
             losses[tag] = {'task_loss_after_%d_steps' % (args.warmup + args.steps): last if last is not None else first_loss()}
         return max_over_ranks(ms), ktimes, ops.launch_count()
@@ -552,9 +580,14 @@ def main():
     ap.add_argument('--no-ddp-check', action='store_true', help='N > 1: skip the data-parallel parity check')
     ap.add_argument('--ref-device', type=str, default='cpu', choices=['cpu', 'cuda'],
                     help='--impl reference only: cuda = the oracle port with stock PyTorch ops on cuda:0 (informational)')
+    ap.add_argument('--dump-outputs', type=str, default=None, metavar='DIR',
+                    help='after the timed steps, write what their last step computed (meters, model state) as '
+                         'DIR/<name>.npy, at most 64 MB; see dump_outputs()')
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == 'engine':
         args.warmup = 3
+    if args.impl == 'reference' and args.dump_outputs:
+        ap.error('--dump-outputs writes what the engine computed; --impl reference has no engine outputs')
     if args.impl == 'reference':
         run_reference(args)
     else:

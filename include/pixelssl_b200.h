@@ -226,12 +226,15 @@ typedef struct {
 int pxl_conv_tc_launch_ex(const pxl_conv_geom* geom_host, const int* taps_dydx_host, const pxl_conv_tc_ext* ext_host,
                           const float* in_hi, const float* in_lo, const float* w_hi, const float* w_lo,
                           const float* bias, float* out, void* stream);
-/* tcgen05 wgrad (accumulates into dw): both operands MN-major via TMA, split over the pixel range,
- * fp32 RED epilogue.  Same precision / operand convention as pxl_conv_tc_launch; needs mul == div == 1,
- * Cin % 32 == 0 and ldo % 32 == 0. */
+/* tcgen05 wgrad (accumulates into dw): both operands MN-major via TMA, split over the pixel range.  Every split
+ * writes its tile into its own slot of the DEVICE workspace ws, and the slots are then added into dw in split order,
+ * so dw is the same in every run.  ws holds at least pxl_conv_wgrad_workspace_floats(geom, taps) floats and must not
+ * be used by another stream until this launch's work on `stream` is done.  Same precision / operand convention as
+ * pxl_conv_tc_launch; needs mul == div == 1, Cin % 32 == 0 and ldo % 32 == 0. */
+int64_t pxl_conv_wgrad_workspace_floats(const pxl_conv_geom* geom_host, const int* taps_dydx_host);
 int pxl_conv_wgrad_tc_launch(const pxl_conv_geom* geom_host, const int* taps_dydx_host, const float* in_hi,
                              const float* in_lo, const float* dy_hi, const float* dy_lo, float* dw,
-                             void* stream);
+                             float* ws, int64_t ws_floats, void* stream);
 /* ---- fp16 pairs: the operand format of the kind::f16 tcgen05 path (csrc/h16_prep.cu) -------------------------
  * x*s = hi + lo, hi = fp16(x*s), lo = fp16(x*s - hi), s a power of two.  precision 3 ("f16x3"): hi*hi + lo*hi +
  * hi*lo in fp32 (products good to ~2^-21: fp32-grade, like 3xTF32, at twice its MMA rate); precision 4 ("f16"):
@@ -244,7 +247,7 @@ int pxl_conv_h16_launch(const pxl_conv_geom* geom_host, const int* taps_dydx_hos
                         const float* bias, float* out, void* stream);
 int pxl_conv_wgrad_h16_launch(const pxl_conv_geom* geom_host, const int* taps_dydx_host, const void* in_hi,
                               const void* in_lo, const void* dy_hi, const void* dy_lo, float* dw, float out_scale,
-                              const float* out_scale_dev, void* stream);
+                              const float* out_scale_dev, float* ws, int64_t ws_floats, void* stream);
 /* x -> (hi, lo).  slot == NULL: fixed `scale`.  slot != NULL (DEVICE float[4], zeroed, then filled by
  * pxl_h16_absmax on the same stream): s = 2^(target_log2 - ceil(log2 absmax)); the kernel stores s in slot[0] and
  * 1/s in slot[1] (what out_scale_dev points at).  lo nullable; n % 4 == 0.  Out-of-range values saturate at

@@ -509,6 +509,73 @@ def golden_input(pixelssl, sseg_proxy):
     print('input_pipeline.npz written:', {k: v.shape for k, v in out.items() if k.startswith(('x', 'y'))})
 
 
+def golden_val_prehandle(pixelssl, sseg_proxy):
+    """Validation input pipeline (task/sseg/data.py ``_val_prehandle``: optional FixedScaleResize + Normalize +
+    ToTensor) on the inputs of tests/test_oracle_golden.py."""
+    import types
+    import data as sseg_data
+    from PIL import Image
+    sys.path.insert(0, os.path.join(ROOT, 'tests'))
+    import test_oracle_golden as T
+    out = {}
+    for k, (h, w, size, rescaling) in enumerate(T.VAL_PREHANDLE_CASES):
+        img, lab = T.val_prehandle_inputs(h, w)
+        fake = types.SimpleNamespace(args=types.SimpleNamespace(val_rescaling=rescaling, im_size=size),
+                                     IMAGE=sseg_data.PascalVocDataset.IMAGE, LABEL=sseg_data.PascalVocDataset.LABEL)
+        x, y = sseg_data.PascalVocDataset._val_prehandle(fake, Image.fromarray(img), Image.fromarray(lab))
+        out['x%d' % k], out['y%d' % k] = x.numpy(), y.numpy()
+    np.savez_compressed(os.path.join(OUT, 'val_prehandle.npz'), **out)
+    print('val_prehandle.npz written:', {k: v.shape for k, v in out.items()})
+
+
+def golden_host(pixelssl, sseg_proxy):
+    """Host-side API of the reference, as tests/test_host_cpu.py compares the engine with it: algorithm registry and
+    sampler stream, task-model state_dict layouts and LR groups, checkpoint keys, parser tables, LR trajectories,
+    constructor argument checks, TaskFunc shape hooks and optimizer hyper-parameters."""
+    import argparse
+    import gzip
+    import importlib
+    import json
+    import func as sseg_func
+    import model as sseg_model
+    from pixelssl import runner as ref_runner
+    from pixelssl.nn import data as ref_data, lrer as ref_lrer, optimizer as ref_optimizer
+    sys.path.insert(0, os.path.join(ROOT, 'tests'))
+    import test_host_cpu as T
+    np.random.seed(5)
+    out = {'register': {'ssl_algorithms': list(pixelssl.ssl_algorithm.SSL_ALGORITHMS),
+                        'sampler_seed5': [list(map(int, b)) for b in ref_data.TwoStreamBatchSampler(
+                            list(range(9)), list(range(50, 83)), 2, 3)]}}
+    out['checkpoint_keys'] = {}
+    out['parser_table'] = {}
+    for alg in T.SSL_ALGS:
+        mod = importlib.import_module('pixelssl.ssl_algorithm.' + alg)
+        with open(mod.__file__) as f:
+            out['checkpoint_keys'][alg] = T._checkpoint_keys(f.read())
+        parser = argparse.ArgumentParser()
+        mod.add_parser_arguments(parser)
+        out['parser_table'][alg] = T._parser_table(parser)
+    parser = ref_runner.create_parser('ssl_null')
+    sseg_proxy.add_parser_arguments(parser)
+    out['full_parser_table'] = T._parser_table(parser, option_strings=False)
+    out['lr_trajectory'] = {n: T._lr_trajectory(ref_lrer, n) for n in T.LR_SCHEDULERS}
+    out['constructor_rejects'] = {T._case_id(alg, ov): T._constructor_rejects(
+        importlib.import_module('pixelssl.ssl_algorithm.' + alg), alg, ov) for alg, ov in T._CASES}
+    out['task_func'] = {}
+    for arch in ('deeplabv2', 'pspnet'):
+        tf = sseg_func.task_func()(T._task_func_args(arch))
+        out['task_func'][arch] = dict({h: getattr(tf, h)() for h in T.SHAPE_HOOKS}, METRIC_STR=tf.METRIC_STR)
+    out['optimizer'] = {n: T._optimizer_summary(ref_optimizer, n) for n in ('sgd', 'adam')}
+    with open(os.path.join(OUT, 'reference_host.json'), 'w') as f:
+        json.dump(out, f, sort_keys=True, indent=1)
+        f.write('\n')
+    # the state_dict layouts are ~140 kB of JSON: stored compressed
+    layouts = {'%s-%s' % (n, b): T._task_model_layout(sseg_model, n, b) for n, b in T.TASK_MODELS}
+    with gzip.open(os.path.join(OUT, 'reference_task_models.json.gz'), 'wt') as f:
+        json.dump(layouts, f, sort_keys=True)
+    print('reference_host.json, reference_task_models.json.gz written:', sorted(out))
+
+
 def golden_fp64_mid(size=257):
     """fp64 truth of the mid-size MT step (mt_steps_257.npz): same seeds as golden_mt(size=257, steps=1)."""
     D = torch.float64
@@ -635,9 +702,10 @@ def golden_fp64():
 
 if __name__ == '__main__':
     os.makedirs(OUT, exist_ok=True)
-    torch.set_num_threads(os.cpu_count())
+    torch.set_num_threads(8)                # tests/test_oracle_golden.py GOLDEN_THREADS: fp32 sums depend on it
     pixelssl, sseg_proxy = patch_and_import()
-    which = sys.argv[1:] or ['ops', 'forward', 'mt', 'nullcutmix', 'adv', 's4l', 'gct', 'cct', 'pspnet', 'val', 'input', 'fp64']
+    which = sys.argv[1:] or ['ops', 'forward', 'mt', 'nullcutmix', 'adv', 's4l', 'gct', 'cct', 'pspnet', 'val', 'input',
+                             'valprehandle', 'host', 'fp64']
     if which == ['fp64']:
         golden_fp64()
         sys.exit(0)
@@ -673,5 +741,9 @@ if __name__ == '__main__':
         golden_val(pixelssl, sseg_proxy)
     if 'input' in which:
         golden_input(pixelssl, sseg_proxy)
+    if 'valprehandle' in which:
+        golden_val_prehandle(pixelssl, sseg_proxy)
+    if 'host' in which:
+        golden_host(pixelssl, sseg_proxy)
     if 'fp64' in which:
         golden_fp64()

@@ -63,9 +63,11 @@ SIGNATURES = {
     'pxl_conv_wgrad_nhwc': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), P, P, P, P]),
     'pxl_conv_tc_launch': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), P, P, P, P, P, P, P]),
     'pxl_conv_tc_launch_ex': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), ctypes.POINTER(ConvTcExt), P, P, P, P, P, P, P]),
-    'pxl_conv_wgrad_tc_launch': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), P, P, P, P, P, P]),
+    'pxl_conv_wgrad_workspace_floats': (c_int64, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int)]),
+    'pxl_conv_wgrad_tc_launch': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), P, P, P, P, P, P, c_int64, P]),
     'pxl_conv_h16_launch': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), ctypes.POINTER(ConvTcExt), P, P, P, P, P, P, P]),
-    'pxl_conv_wgrad_h16_launch': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), P, P, P, P, P, c_float, P, P]),
+    'pxl_conv_wgrad_h16_launch': (c_int, [ctypes.POINTER(ConvGeom), ctypes.POINTER(c_int), P, P, P, P, P, c_float, P, P, c_int64,
+                                          P]),
     'pxl_h16_split': (c_int, [P, P, P, c_int64, c_float, P, c_int, P]),
     'pxl_h16_absmax': (c_int, [P, c_int64, P, P]),
     'pxl_h16_sat_counter': (c_void_p, []),

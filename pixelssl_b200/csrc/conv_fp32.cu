@@ -418,9 +418,12 @@ extern "C" int pxl_conv_transpose_weights_batched(const float* src_base, float* 
 
 // ------------------------------------------------------------------------------------------
 // bias gradient: dbias[co] (+)= sum_rows dy[row*ldo + co]
+// Two passes in a fixed order, so the result is the same in every run: each CTA of the first sums its row block into
+// one partial per channel, the second adds the partials in row-block order.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-bias_grad_kernel(const float* __restrict__ dy, int64_t rows, int Cout, int ldo, int64_t rowsPerBlock, float* __restrict__ dbias) {
+bias_grad_partial_kernel(const float* __restrict__ dy, int64_t rows, int Cout, int ldo, int64_t rowsPerBlock,
+                         float* __restrict__ partial) {
     // thread (c = tid % 32, r = tid / 32); Cout <= 32 per grid.y slice
     const int c = blockIdx.y * 32 + (threadIdx.x & 31), rl = threadIdx.x >> 5;
     const int64_t r0 = (int64_t)blockIdx.x * rowsPerBlock, r1 = min(rows, r0 + rowsPerBlock);
@@ -434,8 +437,16 @@ bias_grad_kernel(const float* __restrict__ dy, int64_t rows, int Cout, int ldo, 
         float t = 0.f;
 #pragma unroll
         for (int i = 0; i < 8; ++i) t += sm[i][threadIdx.x & 31];
-        atomicAdd(dbias + c, t);
+        partial[(int64_t)blockIdx.x * Cout + c] = t;
     }
+}
+
+__global__ void bias_grad_sum_kernel(const float* __restrict__ partial, int nblocks, int Cout, float* __restrict__ dbias) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= Cout) return;
+    float t = 0.f;
+    for (int b = 0; b < nblocks; ++b) t += partial[(int64_t)b * Cout + c];
+    dbias[c] += t;
 }
 
 extern "C" int pxl_bias_grad(const float* dy, int64_t rows, int Cout, int ldo, float* dbias, int accumulate, void* stream) {
@@ -447,10 +458,17 @@ extern "C" int pxl_bias_grad(const float* dy, int64_t rows, int Cout, int ldo, f
     }
     int64_t rb = pxl_cdiv(rows, PXL_NUM_SMS * 4);
     if (rb < 64) rb = 64;
-    dim3 grid((unsigned)pxl_cdiv(rows, rb), (unsigned)pxl_cdiv(Cout, 32));
-    bias_grad_kernel<<<grid, 256, 0, st>>>(dy, rows, Cout, ldo, rb, dbias);
+    const int nblocks = (int)pxl_cdiv(rows, rb);
+    float* partial = nullptr;         // stream-ordered scratch: launches on other streams get their own
+    cudaError_t e = cudaMallocAsync((void**)&partial, sizeof(float) * (size_t)nblocks * Cout, st);
+    if (e != cudaSuccess) return (int)e;
+    dim3 grid((unsigned)nblocks, (unsigned)pxl_cdiv(Cout, 32));
+    bias_grad_partial_kernel<<<grid, 256, 0, st>>>(dy, rows, Cout, ldo, rb, partial);
     PXL_CHECK_LAUNCH();
-    return 0;
+    bias_grad_sum_kernel<<<(unsigned)pxl_cdiv(Cout, 128), 128, 0, st>>>(partial, nblocks, Cout, dbias);
+    PXL_CHECK_LAUNCH();
+    e = cudaFreeAsync(partial, st);
+    return e == cudaSuccess ? 0 : (int)e;
 }
 
 // ------------------------------------------------------------------------------------------

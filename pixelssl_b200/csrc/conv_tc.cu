@@ -169,14 +169,6 @@ __device__ __forceinline__ void tma_store_4d(const void* src, const CUtensorMap*
         ::"l"(map), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
         : "memory");
 }
-// TMA reduce-add: global[box] += shared[box] (fp32), performed by the L2 - the split-K accumulation of the wgrad
-// kernel without one RED instruction per element
-__device__ __forceinline__ void tma_reduce_add_3d(const void* src, const CUtensorMap* map, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];"
-        ::"l"(map), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
 // out[box] += shared[box] (fp32): lets a dgrad launch add its result into a tensor that already holds another
 // gradient (the residual branch of a bottleneck), instead of a separate elementwise add over both tensors
 __device__ __forceinline__ void tma_reduce_add_4d(const void* src, const CUtensorMap* map, int c0, int c1, int c2, int c3) {
@@ -1601,7 +1593,9 @@ extern "C" int pxl_conv_tc_impl(const pxl_conv_geom* g, const int* taps, const f
 // SWIZZLE_128B_ATOM_32B slab; 4 slabs of dY (128 co) and BN/32 slabs of X (tap-shifted, OOB zero-filled)
 // form a stage.  Each tcgen05.mma.kind::tf32 consumes 8 pixel rows (one 1024-B swizzle atom per
 // slab).  Rows between BW*BH and the 8-aligned allocation are zeroed once and never written.
-// The pixel range is split over gridDim.z CTAs; the epilogue adds the tile into dW with fp32 RED.
+// The pixel range is split over gridDim.z CTAs.  Each writes its tile into its own slot of a workspace
+// [split][Cout][taps][Cin]; wg_slot_sum_kernel then adds the slots into dW in split order, so dW does not depend on
+// the order in which the CTAs finish (fp32 adds from different CTAs in arrival order would make every run differ).
 // ==========================================================================================
 struct WgParams {
     int Cin, Cout, ldo, ntaps;
@@ -1612,7 +1606,8 @@ struct WgParams {
     int f16;           // fp16 operands (kind::f16): 64-channel slabs, 16 pixel rows per MMA, plain SWIZZLE_128B
     int slab_ch;       // channels per 128-byte slab row: 32 (tf32) or 64 (fp16)
     float out_scale;   // the tile is multiplied by this (and by *oscale_ptr) before it is added into dW
-    int tma_red;       // epilogue: stage 32-column slabs in the drained ring and add them into dW with TMA reduce
+    int tma_red;       // epilogue: stage 32-column slabs in the drained ring and TMA-store them into the slot
+                       // (PXL_WG_TMA_REDUCE=0: plain stores; the name dates from the reduce-add epilogue)
     int tiles_ci, ktiles_per_cta, ktiles_total;
     short dy[PXL_MAX_TAPS], dx[PXL_MAX_TAPS];
 };
@@ -1648,7 +1643,7 @@ __global__ void __launch_bounds__(320, 1)
 conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_constant__ CUtensorMap mapDyLo,
                      const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapXLo,
                      const __grid_constant__ CUtensorMap mapDw,
-                     const WgParams p, float* __restrict__ dw, int* __restrict__ err_flag,
+                     const WgParams p, float* __restrict__ ws, int* __restrict__ err_flag,
                      const float* __restrict__ oscale_ptr) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ uint64_t full_bar[8], empty_bar[8], ready_bar[8], acc_bar;
@@ -1811,7 +1806,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_con
             if (ok) {
                 const int used = iters < p.nacc ? iters : p.nacc;
                 const float osc = p.out_scale * (oscale_ptr ? __ldg(oscale_ptr) : 1.f);
-                float* drow = dw + ((int64_t)co * p.ntaps + tap) * p.Cin;
+                float* drow = ws + (((int64_t)blockIdx.z * p.Cout + co) * p.ntaps + tap) * p.Cin;
                 const int r = q * 32 + lane;
                 const int et = threadIdx.x - 64;
                 uint32_t sc = 0;
@@ -1827,7 +1822,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_con
                     }
                     if (p.tma_red) {
                         // the operand ring is drained (acc_bar): two 16 KB slabs of it stage the tile, 128 rows (co) x
-                        // 32 floats (ci) in the 128B-swizzled layout, and the TMA unit adds them into dW
+                        // 32 floats (ci) in the 128B-swizzled layout, and the TMA unit stores them into the slot
                         const uint32_t b = sc & 1u;
                         if (et == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
                         asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -1838,7 +1833,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_con
                         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                         asm volatile("bar.sync 1, 128;" ::: "memory");
                         if (et == 0) {
-                            tma_reduce_add_3d(smem + (size_t)b * 16384, &mapDw, ci0 + j, tap, co0);
+                            tma_store_4d(smem + (size_t)b * 16384, &mapDw, ci0 + j, tap, co0, blockIdx.z);
                             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                         }
                         ++sc;
@@ -1848,7 +1843,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapDy, const __grid_con
 #pragma unroll
                     for (int c = 0; c < 32; ++c) {
                         const int ci = ci0 + j + c;
-                        if (ci < p.Cin) atomicAdd(drow + ci, v[c] * osc);
+                        if (ci < p.Cin) drow[ci] = v[c] * osc;
                     }
                 }
                 if (p.tma_red && et == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
@@ -1895,35 +1890,57 @@ static void pick_ktile(int OH, int OW, bool flat, int maxrows, int& BW, int& BH,
     }
 }
 
+// ws_need != NULL: only report the workspace size (split * Cout * taps * Cin floats) the launch would need
 static int conv_wgrad_tc_core(const pxl_conv_geom* g, const int* taps, const void* in_hi, const void* in_lo,
                               const void* dy_hi, const void* dy_lo, float* dw, float out_scale, const float* oscale_ptr,
-                              void* stream);
+                              float* ws, int64_t ws_floats, int64_t* ws_need, void* stream);
+
+// dw[i] += slot[0][i] + slot[1][i] + ... in split order (n floats per slot)
+__global__ void __launch_bounds__(256)
+wg_slot_sum_kernel(const float* __restrict__ ws, float* __restrict__ dw, int64_t n, int split) {
+    PXL_PDL_SYNC();
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        float s = __ldg(ws + i);
+        for (int z = 1; z < split; ++z) s += __ldg(ws + (int64_t)z * n + i);
+        dw[i] += s;
+    }
+}
+
+extern "C" int64_t pxl_conv_wgrad_workspace_floats(const pxl_conv_geom* g, const int* taps) {
+    int64_t need = 0;
+    const int rc = conv_wgrad_tc_core(g, taps, nullptr, nullptr, nullptr, nullptr, nullptr, 1.f, nullptr, nullptr, 0, &need, nullptr);
+    return rc ? (int64_t)rc : need;
+}
 
 extern "C" int pxl_conv_wgrad_tc_launch(const pxl_conv_geom* g, const int* taps, const float* in_hi, const float* in_lo,
-                                        const float* dy_hi, const float* dy_lo, float* dw, void* stream) {
+                                        const float* dy_hi, const float* dy_lo, float* dw, float* ws, int64_t ws_floats,
+                                        void* stream) {
     if (g && g->precision > 2) return PXL_ERR_BAD_ARG;      // fp16 operands go through pxl_conv_wgrad_h16_launch
-    return conv_wgrad_tc_core(g, taps, in_hi, in_lo, dy_hi, dy_lo, dw, 1.f, nullptr, stream);
+    return conv_wgrad_tc_core(g, taps, in_hi, in_lo, dy_hi, dy_lo, dw, 1.f, nullptr, ws, ws_floats, nullptr, stream);
 }
 
 // fp16-pair operands; dw += out_scale * (*out_scale_dev) * sum(dy * x)
 extern "C" int pxl_conv_wgrad_h16_launch(const pxl_conv_geom* g, const int* taps, const void* in_hi, const void* in_lo,
                                          const void* dy_hi, const void* dy_lo, float* dw, float out_scale,
-                                         const float* out_scale_dev, void* stream) {
+                                         const float* out_scale_dev, float* ws, int64_t ws_floats, void* stream) {
     if (!g || (g->precision != 3 && g->precision != 4)) return PXL_ERR_BAD_ARG;
-    return conv_wgrad_tc_core(g, taps, in_hi, in_lo, dy_hi, dy_lo, dw, out_scale != 0.f ? out_scale : 1.f, out_scale_dev, stream);
+    return conv_wgrad_tc_core(g, taps, in_hi, in_lo, dy_hi, dy_lo, dw, out_scale != 0.f ? out_scale : 1.f, out_scale_dev,
+                              ws, ws_floats, nullptr, stream);
 }
 
 static int conv_wgrad_tc_core(const pxl_conv_geom* g, const int* taps, const void* in_hi, const void* in_lo,
                               const void* dy_hi, const void* dy_lo, float* dw, float out_scale, const float* oscale_ptr,
-                              void* stream) {
-    if (!g || !taps || !in_hi || !dy_hi || !dw) return PXL_ERR_BAD_ARG;
+                              float* ws, int64_t ws_floats, int64_t* ws_need, void* stream) {
+    if (!g || !taps) return PXL_ERR_BAD_ARG;
+    if (!ws_need && (!in_hi || !dy_hi || !dw || !ws)) return PXL_ERR_BAD_ARG;
     if (g->div != 1 || (g->mul != 1 && g->mul != 2)) return PXL_ERR_UNSUPPORTED;   // stride 2 via TMA traversal stride
     const int f16 = g->precision >= 3 ? 1 : 0;
     const int slab_ch = f16 ? 64 : 32;
     if (g->Cin % slab_ch != 0 || g->ldo % slab_ch != 0 || g->ntaps > PXL_MAX_TAPS) return PXL_ERR_UNSUPPORTED;
     const int nsplit = (g->precision == 2 || g->precision == 3) ? 3 : 1;
-    if (nsplit == 3 && ((in_lo == nullptr) != (dy_lo == nullptr))) return PXL_ERR_BAD_ARG;
-    if (f16 && nsplit == 3 && !in_lo) return PXL_ERR_BAD_ARG;
+    if (!ws_need && nsplit == 3 && ((in_lo == nullptr) != (dy_lo == nullptr))) return PXL_ERR_BAD_ARG;
+    if (!ws_need && f16 && nsplit == 3 && !in_lo) return PXL_ERR_BAD_ARG;
     const int inkernel = (!f16 && nsplit == 3 && !in_lo) ? 1 : 0;         // in_hi / dy_hi then hold the raw fp32 tensors
     const bool flat = (g->ntaps == 1 && taps[0] == 0 && taps[1] == 0 && g->OH == g->H && g->OW == g->W && g->mul == 1);
     WgParams p;
@@ -1969,7 +1986,7 @@ static int conv_wgrad_tc_core(const pxl_conv_geom* g, const int* taps, const voi
     if (p.stages < 2) return PXL_ERR_UNSUPPORTED;
     p.ktiles_total = p.N * p.tilesH * p.tilesW;
     // split the pixel range: enough CTAs to fill the GPU, and at most ~4096 pixel rows per CTA so the
-    // truncating TMEM accumulation stays at fp32 level (the cross-CTA RED adds round to nearest)
+    // truncating TMEM accumulation stays at fp32 level (the per-split slots are summed with round to nearest)
     const int64_t base_ctas = (int64_t)tiles_co * p.tiles_ci * g->ntaps;
     int64_t by_rows = pxl_cdiv((int64_t)p.ktiles_total * p.rows_alloc, 4096);
     if (by_rows < 1) by_rows = 1;
@@ -1991,6 +2008,11 @@ static int conv_wgrad_tc_core(const pxl_conv_geom* g, const int* taps, const voi
     if (split > 65535) split = 65535;
     p.ktiles_per_cta = (int)pxl_cdiv(p.ktiles_total, split);
     split = pxl_cdiv(p.ktiles_total, p.ktiles_per_cta);
+    // every CTA writes its whole tile into the slot of its pixel range (each slot element is written by exactly one
+    // CTA, so the slots need no clearing); the caller owns the workspace, one per stream
+    const int64_t n = (int64_t)g->Cout * g->ntaps * g->Cin;
+    if (ws_need) { *ws_need = split * n; return 0; }
+    if (ws_floats < split * n) return PXL_ERR_BAD_ARG;
 
     CUtensorMap mDy, mDyLo, mX, mXLo;
     int rc = make_act_map_strided(&mDy, dy_hi, g->ldo, mapW, mapH, mapN, p.BW, p.BH, 1, f16);
@@ -2016,24 +2038,29 @@ static int conv_wgrad_tc_core(const pxl_conv_geom* g, const int* taps, const voi
         attr = true;
     }
     const size_t smem = (size_t)p.stages * stage_bytes + 1024;
-    // dW [Cout][taps][Cin] as a 3-D tensor (Cin, taps, Cout): box {32, 1, 128}, 128-byte swizzle, fp32 reduce-add target
+    // the slots [split][Cout][taps][Cin] as a 4-D tensor (Cin, taps, Cout, split): box {32, 1, 128, 1}, 128-byte swizzle
     static int cfg_wg_red = -1;
     if (cfg_wg_red < 0) { const char* e = getenv("PXL_WG_TMA_REDUCE"); cfg_wg_red = e ? atoi(e) : 1; }
     CUtensorMap mDw = mDy;
     p.tma_red = 0;
-    if (cfg_wg_red && (g->Cin % 4) == 0 && ((uintptr_t)dw % 16) == 0 && (size_t)p.stages * stage_bytes >= 32768) {
+    if (cfg_wg_red && (g->Cin % 4) == 0 && ((uintptr_t)ws % 16) == 0 && (size_t)p.stages * stage_bytes >= 32768) {
         EncodeTiledFn enc = get_encode();
-        cuuint64_t dims[3] = {(cuuint64_t)g->Cin, (cuuint64_t)g->ntaps, (cuuint64_t)g->Cout};
-        cuuint64_t strides[2] = {(cuuint64_t)g->Cin * 4, (cuuint64_t)g->ntaps * g->Cin * 4};
-        cuuint32_t box[3] = {32, 1, 128};
-        cuuint32_t es[3] = {1, 1, 1};
-        if (enc && enc(&mDw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*)dw, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+        cuuint64_t dims[4] = {(cuuint64_t)g->Cin, (cuuint64_t)g->ntaps, (cuuint64_t)g->Cout, (cuuint64_t)split};
+        cuuint64_t strides[3] = {(cuuint64_t)g->Cin * 4, (cuuint64_t)g->ntaps * g->Cin * 4, (cuuint64_t)n * 4};
+        cuuint32_t box[4] = {32, 1, 128, 1};
+        cuuint32_t es[4] = {1, 1, 1, 1};
+        if (enc && enc(&mDw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void*)ws, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
             p.tma_red = 1;
     }
     dim3 grid((unsigned)(tiles_co * p.tiles_ci), (unsigned)g->ntaps, (unsigned)split);
     cudaError_t le = pxl_launch_pdl(conv_wgrad_tc_kernel, grid, dim3(inkernel ? 320 : 192), smem, (cudaStream_t)stream, mDy, mDyLo, mX, mXLo,
-                                    mDw, p, dw, g_err_flag, oscale_ptr);
+                                    mDw, p, ws, g_err_flag, oscale_ptr);
+    if (le != cudaSuccess) return (int)le;
+    PXL_CHECK_LAUNCH();
+    int blocks = (int)(pxl_cdiv(n, 256) < PXL_NUM_SMS * 8 ? pxl_cdiv(n, 256) : PXL_NUM_SMS * 8);
+    le = pxl_launch_pdl(wg_slot_sum_kernel, dim3(blocks), dim3(256), 0, (cudaStream_t)stream,
+                        (const float*)ws, dw, n, (int)split);
     if (le != cudaSuccess) return (int)le;
     PXL_CHECK_LAUNCH();
     return 0;
@@ -2043,5 +2070,13 @@ extern "C" int pxl_conv_wgrad_tc_impl(const pxl_conv_geom* g, const int* taps, c
                                       float* dw, void* stream) {
     if (!g) return PXL_ERR_BAD_ARG;
     if (g->precision == 2) return PXL_ERR_UNSUPPORTED;     // needs split operands: pxl_conv_wgrad_tc_launch
-    return pxl_conv_wgrad_tc_launch(g, taps, in, nullptr, dy, nullptr, dw, stream);
+    // this entry point takes no workspace: a stream-ordered one for this launch only
+    const int64_t need = pxl_conv_wgrad_workspace_floats(g, taps);
+    if (need < 0) return (int)need;
+    float* ws = nullptr;
+    cudaError_t e = cudaMallocAsync((void**)&ws, (size_t)need * sizeof(float), (cudaStream_t)stream);
+    if (e != cudaSuccess) return (int)e;
+    const int rc = pxl_conv_wgrad_tc_launch(g, taps, in, nullptr, dy, nullptr, dw, ws, need, stream);
+    e = cudaFreeAsync(ws, (cudaStream_t)stream);
+    return rc ? rc : (int)e;
 }

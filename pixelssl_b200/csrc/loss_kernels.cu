@@ -15,7 +15,8 @@ extern "C" int pxl_pdl_enabled_(void) {
     if (v < 0) { const char* e = getenv("PXL_PDL"); v = e ? (atoi(e) != 0) : 1; }
     return v;
 }
-extern "C" int pxl_abi_version(void) { return 2; }   // 2: relu_mask argument of the pxl_bn_*_h16 entry points
+// 2: relu_mask argument of the pxl_bn_*_h16 entry points; 3: caller-provided workspace of the wgrad launches
+extern "C" int pxl_abi_version(void) { return 3; }
 extern "C" int64_t pxl_launch_count(void) { return g_launches; }
 extern "C" void pxl_reset_launch_count(void) { g_launches = 0; }
 

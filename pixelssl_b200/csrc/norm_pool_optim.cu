@@ -695,17 +695,22 @@ extern "C" int pxl_maxpool3x3s2_fwd(const float* x, float* y, int N, int H, int 
     return 0;
 }
 
+// One launch per parity class (oy % 2, ox % 2) of the output windows: 3x3 windows at stride 2 whose rows (columns)
+// have the same parity do not overlap, so within a launch every dx element receives at most one gradient and the four
+// launches add them in a fixed order (atomics in arrival order would make the sums differ from run to run).
 __global__ void __launch_bounds__(256)
 maxpool_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, float* __restrict__ dx,
-                   int N, int H, int W, int C, int OH, int OW) {
-    const int64_t total = (int64_t)N * OH * OW * C;
+                   int N, int H, int W, int C, int OH, int OW, int py, int px) {
+    const int PH = (OH - py + 1) / 2, PW = (OW - px + 1) / 2;
+    const int64_t total = (int64_t)N * PH * PW * C;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
-        const int c = (int)(i % C);
-        int64_t p = i / C;
-        const int ox = (int)(p % OW); p /= OW;
-        const int oy = (int)(p % OH);
-        const int n = (int)(p / OH);
+    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < total; j += stride) {
+        const int c = (int)(j % C);
+        int64_t p = j / C;
+        const int ox = 2 * (int)(p % PW) + px; p /= PW;
+        const int oy = 2 * (int)(p % PH) + py;
+        const int n = (int)(p / PH);
+        const int64_t i = ((int64_t)(n * OH + oy) * OW + ox) * C + c;
         float m = -CUDART_INF_F;
         int64_t arg = -1;
 #pragma unroll
@@ -721,7 +726,7 @@ maxpool_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, fl
                 if (arg < 0 || v > m || isnan(v)) { m = v; arg = idx; }
             }
         }
-        if (arg >= 0) atomicAdd(dx + arg, __ldg(dy + i));
+        if (arg >= 0) dx[arg] += __ldg(dy + i);
     }
 }
 
@@ -732,10 +737,14 @@ extern "C" int pxl_maxpool3x3s2_bwd(const float* x, const float* y, const float*
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaMemsetAsync(dx, 0, sizeof(float) * (size_t)N * H * W * C, st);
     if (e != cudaSuccess) return (int)e;
-    const int64_t total = (int64_t)N * OH * OW * C;
-    int blocks = (int)(pxl_cdiv(total, 256) < PXL_NUM_SMS * 16 ? pxl_cdiv(total, 256) : PXL_NUM_SMS * 16);
-    maxpool_bwd_kernel<<<blocks, 256, 0, st>>>(x, dy, dx, N, H, W, C, OH, OW);
-    PXL_CHECK_LAUNCH();
+    for (int cls = 0; cls < 4; ++cls) {
+        const int py = cls >> 1, px = cls & 1;
+        const int64_t total = (int64_t)N * ((OH - py + 1) / 2) * ((OW - px + 1) / 2) * C;
+        if (total <= 0) continue;
+        int blocks = (int)(pxl_cdiv(total, 256) < PXL_NUM_SMS * 16 ? pxl_cdiv(total, 256) : PXL_NUM_SMS * 16);
+        maxpool_bwd_kernel<<<blocks, 256, 0, st>>>(x, dy, dx, N, H, W, C, OH, OW, py, px);
+        PXL_CHECK_LAUNCH();
+    }
     return 0;
 }
 

@@ -90,17 +90,18 @@ __device__ __forceinline__ void y_support(int i, int h, int H, float sh, bool ac
 //   * the ~2/sh contributing high-res rows are staged G at a time by the whole CTA (coalesced loads,
 //     G*W/128 independent loads per thread), stored at x + x/R so that lanes walking supports that
 //     start R apart hit distinct banks;
-//   * work item = (staged row g, column j): a SUP-long dot product from shared memory, one shared
-//     atomicAdd per item.
+//   * work item = (staged row g, column j): a SUP-long dot product from shared memory, added into the
+//     accumulator row of slot g (the same thread owns item (g, j) in every group, so no atomics); the G slot
+//     rows are summed in slot order at the end - the same result every run.
 template <bool NHWC>
 __global__ void __launch_bounds__(128)
 bilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, int C, int h, int w, int H, int W,
                     float sh, float sw, bool ac, int ldc, int R, int rowbuf, int SUP, int G) {
     extern __shared__ float smem[];
     const int wpad = (w + 31) & ~31;
-    float* acc = smem;                                   // [wpad]
-    int4* meta = reinterpret_cast<int4*>(smem + wpad);   // [wpad] {xlo, count, padded start, xlo % R}
-    float* wtab = smem + wpad + 4 * wpad;                // [w][SUP]
+    float* acc = smem;                                   // [G][wpad]
+    int4* meta = reinterpret_cast<int4*>(smem + G * wpad);   // [wpad] {xlo, count, padded start, xlo % R}
+    float* wtab = smem + G * wpad + 4 * wpad;            // [w][SUP]
     float* rb = wtab + (((size_t)w * SUP + 3) & ~(size_t)3);   // [G][rowbuf]
     const int i = blockIdx.x, b = blockIdx.z;
 
@@ -145,7 +146,7 @@ bilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, int
     y_support(i, h, H, sh, ac, ylo, yhi);
     for (int c = blockIdx.y; c < C; c += gridDim.y) {
     __syncthreads();                                      // tables ready / previous channel written out
-    for (int j = threadIdx.x; j < w; j += blockDim.x) acc[j] = 0.f;
+    for (int j = threadIdx.x; j < G * wpad; j += blockDim.x) acc[j] = 0.f;
     const float* gp = gout + ((int64_t)b * C + c) * (int64_t)H * W;
     for (int y0g = ylo; y0g <= yhi; y0g += G) {
         const int rows = min(G, yhi - y0g + 1);
@@ -184,13 +185,15 @@ bilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, int
                 ++pidx;
                 if (++rem == R) { rem = 0; ++pidx; }
             }
-            atomicAdd(acc + j, sacc * wy);
+            acc[g * wpad + j] += sacc * wy;
         }
     }
     __syncthreads();
     for (int j = threadIdx.x; j < w; j += blockDim.x) {
-        if (NHWC) gin[((int64_t)(b * h + i) * w + j) * ldc + c] = acc[j];
-        else gin[(((int64_t)b * C + c) * h + i) * w + j] = acc[j];
+        float s = acc[j];
+        for (int g = 1; g < G; ++g) s += acc[g * wpad + j];
+        if (NHWC) gin[((int64_t)(b * h + i) * w + j) * ldc + c] = s;
+        else gin[(((int64_t)b * C + c) * h + i) * w + j] = s;
     }
     }
 }
@@ -214,12 +217,12 @@ extern "C" int pxl_bilinear_bwd(const float* grad_out, float* grad_in, int n, in
     SUP |= 1;
     const int rowbuf = ((W + W / R + 1) + 31) & ~31;
     const int wpad = (w + 31) & ~31;
-    const size_t fixed = (size_t)wpad * 5 + (((size_t)w * SUP + 3) & ~(size_t)3);
+    const size_t fixed = (size_t)wpad * 4 + (((size_t)w * SUP + 3) & ~(size_t)3);
     const size_t budget = 48 * 1024 / sizeof(float);
-    if (fixed + (size_t)rowbuf > budget) return PXL_ERR_UNSUPPORTED;
-    int G = (int)((budget - fixed) / rowbuf);
+    if (fixed + (size_t)(rowbuf + wpad) > budget) return PXL_ERR_UNSUPPORTED;
+    int G = (int)((budget - fixed) / (rowbuf + wpad));      // per staged row: its buffer and its accumulator row
     if (G > 8) G = 8;
-    const size_t smem = (fixed + (size_t)G * rowbuf) * sizeof(float);
+    const size_t smem = (fixed + (size_t)G * (rowbuf + wpad)) * sizeof(float);
     if (in_nhwc) bilinear_bwd_kernel<true><<<grid, 128, smem, st>>>(grad_out, grad_in, C, h, w, H, W, sh, sw, align_corners != 0, ldc, R, rowbuf, SUP, G);
     else bilinear_bwd_kernel<false><<<grid, 128, smem, st>>>(grad_out, grad_in, C, h, w, H, W, sh, sw, align_corners != 0, C, R, rowbuf, SUP, G);
     PXL_CHECK_LAUNCH();

@@ -652,6 +652,27 @@ def conv_tc_status():
     return int(_lib.load().pxl_conv_tc_status())
 
 
+_wgrad_ws = {}          # (device, stream) -> workspace of the tcgen05 wgrad launches enqueued on that stream
+_wgrad_ws_need = {}     # geometry -> floats it needs
+
+
+def _wgrad_workspace(geom, taps, device, key):
+    """Workspace of one tcgen05 wgrad launch (its per-split dW slots).  One per stream, so that launches on different
+    streams never share slots; a larger request replaces it through torch's caching allocator, which hands the old
+    block out again only after the work already queued on that stream."""
+    need = _wgrad_ws_need.get(key)
+    if need is None:
+        need = int(_lib.load().pxl_conv_wgrad_workspace_floats(ctypes.byref(geom), _ctaps(taps)))
+        if need < 0:
+            raise _lib.PxlError('pxl_conv_wgrad_workspace_floats', need)
+        _wgrad_ws_need[key] = need
+    skey = (device, _stream())
+    ws = _wgrad_ws.get(skey)
+    if ws is None or ws.numel() < need:
+        ws = _wgrad_ws[skey] = torch.empty(need, dtype=torch.float32, device=device)
+    return ws
+
+
 def conv_wgrad_raw(x, dy, dw, taps, N, H, W, Cin, OH, OW, Cout, ldo, mul, div, precision=None):
     """dw[Cout][ntaps][Cin] += ...  (dw must be initialised by the caller)."""
     ntaps = len(taps) // 2
@@ -669,12 +690,14 @@ def conv_wgrad_raw(x, dy, dw, taps, N, H, W, Cin, OH, OW, Cout, ldo, mul, div, p
         if px is not None and pd is not None:
             raise ValueError('at most one operand may carry a device-side scale')
         geom = ConvGeom(N, H, W, Cin, OH, OW, Cout, ldo, mul, div, ntaps, prec)
+        ws = _wgrad_workspace(geom, taps, dw.device, (N, H, W, Cin, OH, OW, Cout, ldo, mul, div, prec, tuple(taps)))
         _timed_call('pxl_conv_wgrad_h16_launch', ctypes.byref(geom), _ctaps(taps), _p(xh.hi), _p(xh.lo), _p(dh.hi), _p(dh.lo),
-                    _p(dw), float(fx * fd), _p(pd if pd is not None else px), _stream(),
+                    _p(dw), float(fx * fd), _p(pd if pd is not None else px), _p(ws), ws.numel(), _stream(),
                     meta=(2.0 * N * OH * OW * Cin * Cout * ntaps, 'wgrad N%d %dx%d Cin%d Cout%d taps%d mul%d' % (N, OH, OW, Cin, Cout, ntaps, mul)))
         return dw
     if prec != 0 and div == 1 and mul in _WGRAD_TC_STRIDES and Cin % 32 == 0 and ldo % 32 == 0:
         geom = ConvGeom(N, H, W, Cin, OH, OW, Cout, ldo, mul, div, ntaps, prec)
+        ws = _wgrad_workspace(geom, taps, dw.device, (N, H, W, Cin, OH, OW, Cout, ldo, mul, div, prec, tuple(taps)))
         if prec == 2:
             if isinstance(x, tuple) != isinstance(dy, tuple):        # mixed: split the raw one too
                 x = x if isinstance(x, tuple) else split_tf32(x)
@@ -682,10 +705,10 @@ def conv_wgrad_raw(x, dy, dw, taps, N, H, W, Cin, OH, OW, Cout, ldo, mul, div, p
             x_hi, x_lo = x if isinstance(x, tuple) else (x, None)     # raw operands: split inside the kernel
             d_hi, d_lo = dy if isinstance(dy, tuple) else (dy, None)
             _timed_call('pxl_conv_wgrad_tc_launch', ctypes.byref(geom), _ctaps(taps), _p(x_hi), _p(x_lo), _p(d_hi), _p(d_lo),
-                        _p(dw), _stream(), meta=(2.0 * N * OH * OW * Cin * Cout * ntaps, 'wgrad(tf32) N%d %dx%d Cin%d Cout%d taps%d' % (N, OH, OW, Cin, Cout, ntaps)))
+                        _p(dw), _p(ws), ws.numel(), _stream(), meta=(2.0 * N * OH * OW * Cin * Cout * ntaps, 'wgrad(tf32) N%d %dx%d Cin%d Cout%d taps%d' % (N, OH, OW, Cin, Cout, ntaps)))
         else:
             _timed_call('pxl_conv_wgrad_tc_launch', ctypes.byref(geom), _ctaps(taps), _p(x), _p(None), _p(dy), _p(None),
-                        _p(dw), _stream(), meta=(2.0 * N * OH * OW * Cin * Cout * ntaps, 'wgrad(tf32) N%d %dx%d Cin%d Cout%d taps%d' % (N, OH, OW, Cin, Cout, ntaps)))
+                        _p(dw), _p(ws), ws.numel(), _stream(), meta=(2.0 * N * OH * OW * Cin * Cout * ntaps, 'wgrad(tf32) N%d %dx%d Cin%d Cout%d taps%d' % (N, OH, OW, Cin, Cout, ntaps)))
         return dw
     if isinstance(x, tuple):
         x = x[0] + x[1]

@@ -245,3 +245,37 @@ def test_checkpoint_roundtrip(eng, tmp_path):
     assert alg2.load_checkpoint() == 3
     for (n1, p1), (n2, p2) in zip(alg.s_model.named_parameters(), alg2.s_model.named_parameters()):
         assert torch.equal(p1, p2), n1
+
+
+def test_wgrad_side_stream_and_repeat_give_identical_step(eng, monkeypatch):
+    """One MT step from the same weights and batch, twice in the default mode and once with the bottleneck wgrads on a
+    side stream (PXL_WGRAD_SIDE_STREAM) while the other wgrads stay on the current stream - each stream with its own
+    wgrad workspace.  Gradients, updated weights and BN running statistics agree bit for bit: the split-K wgrad,
+    max-pool, bilinear and bias-gradient reductions add in a fixed order."""
+    from pixelssl_b200 import ops, runner
+    if ops.get_conv_precision() == ops.PRECISION['fp32']:
+        pytest.skip('the exact-fp32 FFMA wgrad kernels (csrc/conv_fp32.cu) still add their split-K partials with atomics')
+    img, lab = O.synthetic_batch(5, 2, 1, 65, 65)
+    s, t = _state((1, 2)), _state((3, 4))
+
+    def run(side):
+        monkeypatch.setattr(ops, 'WGRAD_SIDE_STREAM', side)
+        monkeypatch.setattr(ops, '_side_streams', {})
+        alg = runner.build_algorithm(runner.build_args(_cfg('ssl_mt', cons_for_labeled=False, cons_scale=1.0,
+                                                            cons_rampup_epochs=1, ema_decay=0.99, batch_size=2,
+                                                            unlabeled_batch_size=1), iters_per_epoch=5))
+        _load(alg.s_model, s)
+        _load(alg.t_model, t)
+        alg._train([((img,), (lab,))], 0)
+        torch.cuda.synchronize()
+        bufs = torch.cat([b.reshape(-1).float() for n, b in alg.s_model.named_buffers() if 'num_batches' not in n])
+        return [alg.s_model.arena.grad.clone(), alg.s_model.arena.data.clone(), bufs], bool(ops._side_streams)
+
+    first, _ = run(False)
+    again, _ = run(False)
+    side, used = run(True)
+    if ops.get_conv_precision() == ops.PRECISION['f16x3']:
+        assert used, 'no wgrad ran on the side stream'
+    for what, a, b, c in zip(('gradients', 'weights', 'BN statistics'), first, again, side):
+        assert torch.equal(a, b), what + ' differ between two default-mode runs'
+        assert torch.equal(a, c), what + ' differ between the default and the side-stream mode'

@@ -13,6 +13,19 @@ from oracle import sseg_oracle as O
 
 G = os.path.join(os.path.dirname(__file__), 'golden')
 
+# Intra-op threads the fixtures were generated with (oracle/make_golden.py).  torch's CPU convolutions block their fp32
+# reductions by thread count, and the deep random-init nets amplify that reassociation noise past the step tolerances
+# below (1 or 4 threads on an 8-core host, 16 on a 16-core one: gradient checksums off by 1e-2 .. 2e-1).
+GOLDEN_THREADS = 8
+
+
+@pytest.fixture(autouse=True)
+def golden_thread_count():
+    saved = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(saved)
+
 
 def load(name):
     return np.load(os.path.join(G, name), allow_pickle=False)
@@ -361,26 +374,25 @@ def test_resize_restatements_are_bit_exact_against_pillow():
         assert np.array_equal(I.resize_nearest(m, ow, oh), np.array(Image.fromarray(m).resize((ow, oh), Image.NEAREST)))
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference'), reason='reference tree only exists in the build container')
-@pytest.mark.parametrize('h,w,size,rescaling', [(37, 53, 33, True), (64, 41, 48, True), (30, 30, 30, True), (45, 70, 0, False)])
-def test_validation_input_pipeline_matches_reference_transforms(h, w, size, rescaling):
-    """_val_prehandle (optional FixedScaleResize + Normalize + ToTensor) against the reference classes, bit for bit."""
-    import sys
-    import types
-    for p in ('/root/reference', '/root/reference/task/sseg'):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import data as sseg_data
-    from PIL import Image
-    from oracle import input_oracle as I
+VAL_PREHANDLE_CASES = [(37, 53, 33, True), (64, 41, 48, True), (30, 30, 30, True), (45, 70, 0, False)]
+
+
+def val_prehandle_inputs(h, w):
     rs = np.random.RandomState(h * 100 + w)
     img = rs.randint(0, 256, (h, w, 3)).astype(np.uint8)
     lab = rs.randint(0, 21, (h, w)).astype(np.uint8)
-    fake = types.SimpleNamespace(args=types.SimpleNamespace(val_rescaling=rescaling, im_size=size),
-                                 IMAGE=sseg_data.PascalVocDataset.IMAGE, LABEL=sseg_data.PascalVocDataset.LABEL)
-    x_ref, y_ref = sseg_data.PascalVocDataset._val_prehandle(fake, Image.fromarray(img), Image.fromarray(lab))
-    x, y = I.val_prehandle(img, lab, size, rescaling)
-    assert np.array_equal(x, x_ref.numpy()) and np.array_equal(y, y_ref.numpy())
+    return img, lab
+
+
+@pytest.mark.parametrize('h,w,size,rescaling', VAL_PREHANDLE_CASES)
+def test_validation_input_pipeline_matches_reference_transforms(h, w, size, rescaling):
+    """_val_prehandle (optional FixedScaleResize + Normalize + ToTensor) against the reference classes, bit for bit
+    (fixture generated by oracle/make_golden.py valprehandle)."""
+    from oracle import input_oracle as I
+    g = load('val_prehandle.npz')
+    k = VAL_PREHANDLE_CASES.index((h, w, size, rescaling))
+    x, y = I.val_prehandle(*val_prehandle_inputs(h, w), size, rescaling)
+    assert np.array_equal(x, g['x%d' % k]) and np.array_equal(y, g['y%d' % k])
 
 
 @pytest.mark.slow
